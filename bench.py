@@ -58,6 +58,8 @@ def parse():
     ap.add_argument("--tf32", action="store_true", help="LightGlue linears as single TF32 (fast mode, not parity-grade)")
     ap.add_argument("--sp-simt", action="store_true", help="SuperPoint convs on fp32 CUDA cores")
     ap.add_argument("--dump-sites", default="", help="write the launch-site profile of one step to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
     return ap.parse_args()
 
 
@@ -101,6 +103,27 @@ class ClockSampler:
                 if v.lower().startswith("active"):
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """One DIR/<name>.npy per output: float32 stays float32, everything else (int32 counts and indices) becomes float64,
+    which holds it exactly.  An output larger than its share of DUMP_BYTES keeps a fixed seeded sample of its rows, listed
+    in DIR/<name>_rows.npy.  The inputs are seeded, so two builds given the same arguments can be compared file by file."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // max(len(arrays), 1)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if a.nbytes > share:
+            keep = max(1, share // max(a.nbytes // len(a), 1))
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            np.save(out_dir / f"{name}_rows.npy", rows.astype(np.float64))
+            a = a[rows]
+        np.save(out_dir / f"{name}.npy", a)
 
 
 def host_threads():
@@ -191,10 +214,12 @@ class Config2:
             return
         from imcui_b200.engine import PairEngine, PairStream
         from imcui_b200.hloc.configs import confs_dict
+        from imcui_b200.utils import synth_weights
         lg_mode = 0 if args.fp32 else (2 if args.tf32 else 1)
         self.pre = dict(confs_dict["extractors"]["superpoint_max"]["preprocessing"])     # grayscale, resize_max 1600, dfactor 8
         self.eng = PairEngine(dev, P, H, W, sp_conf={**SP_CONF, "tensor_cores": not (args.fp32 or args.sp_simt)},
-                              lg_conf={"use_tensor_cores": lg_mode}, frame_shape=(H, W, 3), pre_conf=self.pre)
+                              lg_conf={"use_tensor_cores": lg_mode}, frame_shape=(H, W, 3), pre_conf=self.pre,
+                              sp_state_dict=synth_weights.superpoint_random_weights(0), lg_state_dict=synth_weights.lightglue_random_weights(0))
         self.stream = PairStream(self.eng)
         self.record = self.eng.new_record()
         self.d_batches = [hb.to(dev) for hb in self.h_batches]       # decoded uint8 frames, resident in HBM
@@ -222,6 +247,13 @@ class Config2:
     def d2h_bytes(self):
         return self.stream.d2h_bytes
 
+    def outputs(self):
+        """The match record of the last step (what match_frames_device hands its caller), slots past each pair's match
+        count zeroed."""
+        rec = self.record
+        valid = torch.arange(rec["mconf"].shape[1], device=rec["mconf"].device)[None] < rec["mcount"][:, None]
+        return {k: (v * valid[..., None] if v.dim() == 3 else v * valid if v.shape == valid.shape else v) for k, v in rec.items()}
+
     def stats(self):
         return {"mean_keypoints": float(self.record["n_kpts"].float().mean()), "mean_stop_layer": float(self.record["stop"].float().mean())}
 
@@ -229,7 +261,7 @@ class Config2:
         st = self.stats()
         return {"workload": "SuperPoint+LightGlue, batch=64 synthetic 640x480 pairs per GPU (BASELINE configs[1]); each step starts from the decoded RGB frames "
                             "(GPU gray conversion / normalisation = extract()'s pre-processing) and ends with the matched keypoints in original-frame coordinates",
-                "pairs_per_gpu": self.P, "max_keypoints": 1024, "weights": "superpoint_v1 + GIM SP-LightGlue (real)",
+                "pairs_per_gpu": self.P, "max_keypoints": 1024, "weights": "deterministic synthetic SuperPoint + LightGlue (utils/synth_weights.py)",
                 "lightglue": "depth_confidence 0.95, width_confidence 0.99, CUDA pruning threshold 1536 (reference CUDA semantics)",
                 **st, "stream": f"cycle of {NB} distinct batches dealt round-robin over ranks (seeds 0..{NB * self.P - 1})",
                 "l2": "per-step working set (> 1 GB of activations per 32-image conv pass) >> 126 MB L2, and consecutive steps take different batches; no explicit flush"}
@@ -258,7 +290,7 @@ class Config2:
         import oracle
         from oracle import superpoint as osp
         from oracle.check import to_float
-        ws = oracle.load_weights("superpoint_v1.pt")
+        ws = oracle.synthetic_weights("superpoint")
         img = to_float(self._gray(0, 1)[:1])
         return lambda: osp.forward(ws, img, SP_CONF)
 
@@ -375,6 +407,8 @@ def main():
         counts_log[k] = cfg.step_device(batch_of(Wu + k))
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cfg.outputs() if hasattr(cfg, "outputs") else {"mcount": counts_log[K - 1]})
     per_rank = rank_times(e0.elapsed_time(e1))
     launches = L.lib().imw_launch_count() - l0
     clocks = sampler.stop() if sampler else None

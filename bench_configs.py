@@ -204,7 +204,7 @@ class Config4(_Base):
     cpu_sample_pairs = 2
     workload_desc = ("ALIKED-n16 (RGB 640x480, top-1024 keypoints) -> LightGlue features='aliked' architecture (128-d input_proj, 9 layers) -> "
                      "MAGSAC++ fundamental matrix 3 px / 0.9999 / 10000 on the matched keypoints (BASELINE configs[3]); seeded random ALIKED "
-                     "weights + GIM LightGlue weights with an input_proj FITTED (ridge regression, tools/make_golden.py aliked_lg_case) so that "
+                     "weights + synthetic LightGlue weights (utils/synth_weights.py) with an input_proj FITTED (ridge regression, tools/make_golden.py aliked_lg_case) so that "
                      "the trained matcher sees SuperPoint-like descriptors: no aliked checkpoints offline, yet hundreds of geometrically "
                      "correct matches per pair reach MAGSAC; reference LightGlue semantics (depth 0.95 / width 0.99 / threshold 0.2)")
     dtype = "f32 (ALIKED, CUDA cores), split-fp16 tcgen05 = f32-equivalent (LightGlue), f64 (MAGSAC++ solvers)"
@@ -226,7 +226,7 @@ class Config4(_Base):
             self.h_batches.append(torch.from_numpy(rgb) if self.host_only else _pin(rgb))
         self.asd = synth_weights.aliked_random_weights(0)
         gz = np.load(ROOT / "tests/golden/aliked_lg.npz")    # fitted input_proj (see workload_desc)
-        self.lsd = dict(torch.load(str(ROOT / "weights/superpoint_lightglue.pt"), map_location="cpu"))
+        self.lsd = synth_weights.lightglue_random_weights(0)
         self.lsd["input_proj.weight"], self.lsd["input_proj.bias"] = torch.from_numpy(gz["input_proj_w"]), torch.from_numpy(gz["input_proj_b"])
         if self.host_only:
             return
@@ -334,7 +334,8 @@ class Config1(_Base):
             return
         from imcui_b200.hloc import extractors, matchers
         from imcui_b200.hloc.utils.base_model import dynamic_load
-        self.sp = dynamic_load(extractors, "superpoint")(dict(self.SP)).eval().to(dev)
+        from imcui_b200.utils import synth_weights
+        self.sp = dynamic_load(extractors, "superpoint")({**self.SP, "state_dict": synth_weights.superpoint_random_weights(0)}).eval().to(dev)
         self.nn = dynamic_load(matchers, "nearest_neighbor")({"do_mutual_check": True}).eval().to(dev)
         from imcui_b200.hloc.pipeline import FramePrep
         pre = FramePrep(self.PRE, dev)(self.rgb)
@@ -386,7 +387,7 @@ class Config1(_Base):
         import cv2
         import oracle
         from oracle import matchers as om, superpoint as osp
-        ws = oracle.load_weights("superpoint_v1.pt")
+        ws = oracle.synthetic_weights("superpoint")
         feats = []
         for r in self.rgb:
             g = cv2.cvtColor(r, cv2.COLOR_RGB2GRAY).astype(np.float32)

@@ -20,17 +20,19 @@ LG_CONF_DEFAULT = {"depth_confidence": 0.95, "width_confidence": 0.99, "filter_t
 
 
 class PairEngine:
-    def __init__(self, device, n_pairs, height=480, width=640, sp_conf=None, lg_conf=None, n_layers=9, frame_shape=None, pre_conf=None):
+    def __init__(self, device, n_pairs, height=480, width=640, sp_conf=None, lg_conf=None, n_layers=9, frame_shape=None, pre_conf=None,
+                 sp_state_dict=None, lg_state_dict=None):
         """height/width: size of the network input.  frame_shape (H0, W0[, 3]) + pre_conf (the registry's `preprocessing`
-        dict): decoded frames of that shape are prepared on the device; their prepared size must equal (height, width)."""
+        dict): decoded frames of that shape are prepared on the device; their prepared size must equal (height, width).
+        sp_state_dict / lg_state_dict: in-memory checkpoints (reference key names) instead of weights/*.pt."""
         self.device = torch.device(device)
         self.P, self.H, self.W = n_pairs, height, width
         self.sp_conf = {**SP_CONF_DEFAULT, **(sp_conf or {})}
         self.lg_conf = {**LG_CONF_DEFAULT, **(lg_conf or {})}
         self.n_layers = n_layers
         L.lib()  # fail loudly now if the CUDA library is missing
-        sp_sd = torch.load(str(WEIGHTS_DIR / "superpoint_v1.pt"), map_location="cpu")
-        lg_sd = torch.load(str(WEIGHTS_DIR / "superpoint_lightglue.pt"), map_location="cpu")
+        sp_sd = sp_state_dict if sp_state_dict is not None else torch.load(str(WEIGHTS_DIR / "superpoint_v1.pt"), map_location="cpu")
+        lg_sd = lg_state_dict if lg_state_dict is not None else torch.load(str(WEIGHTS_DIR / "superpoint_lightglue.pt"), map_location="cpu")
         self.sp_w = {k: v.to(self.device) for k, v in ops.sp_pack_weights(sp_sd).items()}
         self.lg_w = {k: v.to(self.device) for k, v in ops.lg_pack_weights(lg_sd, n_layers).items()}
         mk = self.sp_conf["max_keypoints"]

@@ -16,6 +16,7 @@ class SuperPoint(BaseModel):
         "max_keypoints": -1,
         "remove_borders": 4,
         "fix_sampling": False,
+        "state_dict": None,  # B200 engine: in-memory checkpoint (reference key names) instead of model_name
         # B200 engine switch (not in the reference): encoder convs on tcgen05 with split-fp16 operands (2 planes, 3 products)
         # (fp32-equivalent products, needs W % 128 == 0); False = fp32 CUDA-core convs
         "tensor_cores": True,
@@ -27,9 +28,12 @@ class SuperPoint(BaseModel):
         mk = conf["max_keypoints"]
         if mk == 0 or mk < -1:  # superpoint.py:139-141
             raise ValueError('"max_keypoints" must be positive or "-1"')
-        weights_path = self._download_model(
-            repo_id=MODEL_REPO_ID, filename="{}/{}".format("superglue", self.conf["model_name"]))
-        sd = torch.load(str(weights_path), map_location="cpu")
+        sd = conf.get("state_dict")
+        if sd is None:
+            weights_path = self._download_model(
+                repo_id=MODEL_REPO_ID, filename="{}/{}".format("superglue", self.conf["model_name"]))
+            sd = torch.load(str(weights_path), map_location="cpu")
+        self.conf["state_dict"] = None
         for k, v in ops.sp_pack_weights(sd).items():
             self.register_buffer(k, v, persistent=False)
         self._uncapped_cap = 8192

@@ -14,14 +14,18 @@ class SuperGlue(BaseModel):
         "model_name": "superglue_outdoor.pth",
         "sinkhorn_iterations": 100,
         "match_threshold": 0.2,
+        "state_dict": None,  # B200 engine: in-memory checkpoint (reference key names) instead of model_name
         "tensor_cores": True,  # B200 engine switch: True/"3xtf32", "tf32", False (see matchers/lightglue.py)
     }
     required_inputs = ["image0", "keypoints0", "scores0", "descriptors0", "image1", "keypoints1", "scores1", "descriptors1"]
 
     def _init(self, conf):
         assert conf["weights"] in ["indoor", "outdoor"]  # superglue.py:221
-        weights_path = self._download_model(repo_id=MODEL_REPO_ID, filename="{}/{}".format("superglue", self.conf["model_name"]))
-        sd = torch.load(str(weights_path), map_location="cpu")
+        sd = conf.get("state_dict")
+        if sd is None:
+            weights_path = self._download_model(repo_id=MODEL_REPO_ID, filename="{}/{}".format("superglue", self.conf["model_name"]))
+            sd = torch.load(str(weights_path), map_location="cpu")
+        self.conf["state_dict"] = None
         self.bin_score = float(sd["bin_score"])
         for k, v in ops.sg_pack_weights(sd).items():
             self.register_buffer(k.replace(".", "__"), v, persistent=False)

@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import lightglue as olg
-from . import load_weights
+from . import synthetic_weights
 from . import superpoint as osp
 
 LG_CONF_CUDA = {"depth_confidence": 0.95, "width_confidence": 0.99, "filter_threshold": 0.2, "pruning_min_kpts": 1536}
@@ -30,7 +30,7 @@ def to_float(images_u8):
 def oracle_pairs(images_u8, sp_conf, lg_conf=None, weights=None):
     """images_u8 [2n,H,W] uint8 (slot 2p+side) -> list of per-pair dicts
     {kpts0, kpts1 [N,2] f32, scores0/1, matches0 [N0] int64, mscores0, stop}."""
-    ws, wl = weights or (load_weights("superpoint_v1.pt"), load_weights("superpoint_lightglue.pt"))
+    ws, wl = weights or (synthetic_weights("superpoint"), synthetic_weights("lightglue"))
     lg_conf = {**LG_CONF_CUDA, **(lg_conf or {})}
     out = []
     imgs = to_float(images_u8)

@@ -47,7 +47,7 @@ def test_superglue_packing_is_a_relabelling():
     import ctypes
     from imcui_b200 import _lib
     assert ctypes.sizeof(_lib.SGLayer) == 8 * 8 + 8
-    sd = oracle.load_weights("superglue_outdoor.pt")
+    sd = oracle.synthetic_weights("superglue")
     pk = ops.sg_pack_weights(sd)
     x = torch.randn(1, 256, 7)
     ref = torch.nn.functional.conv1d(x, sd["gnn.layers.0.attn.proj.0.weight"], sd["gnn.layers.0.attn.proj.0.bias"]).view(1, 64, 4, 7)
@@ -87,7 +87,7 @@ def test_no_cpu_fallback():
 def test_qkv_permutation_is_a_relabelling():
     from imcui_b200 import ops
     import oracle
-    sd = oracle.load_weights("superpoint_lightglue.pt")
+    sd = oracle.synthetic_weights("lightglue")
     packed = ops.lg_pack_weights(sd)
     w = sd["transformers.0.self_attn.Wqkv.weight"]
     x = torch.randn(5, 256)

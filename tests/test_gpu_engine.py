@@ -32,10 +32,11 @@ def stream():
 def test_engine_default_path_vs_oracle(dev, stream):
     """Keypoint set per image, stop layer per pair, match-F1 and exactness of the match sets."""
     from oracle import check
+    import oracle
     from imcui_b200.engine import PairEngine
     imgs, ref = stream
     P = len(SEEDS)
-    eng = PairEngine(dev, P, 480, 640)       # defaults == what bench.py constructs
+    eng = PairEngine(dev, P, 480, 640, sp_state_dict=oracle.synthetic_weights("superpoint"), lg_state_dict=oracle.synthetic_weights("lightglue"))       # defaults == what bench.py constructs
     assert eng.sp_conf.get("tensor_cores", True) and eng.lg_conf["use_tensor_cores"] == 1
     eng.h_images.copy_(torch.from_numpy(imgs))
     hm, hs, hk, hc, hstop = eng.match_host()
@@ -63,10 +64,11 @@ def test_engine_lightglue_on_oracle_features(dev, stream):
     stop layer identical, matches0 compared index by index; reports the fraction of bit-identical pairs."""
     from oracle.check import compare_pair
     from imcui_b200 import ops
+    import oracle
     from imcui_b200.engine import PairEngine
     _, ref = stream
     P, cap = len(SEEDS), 1024
-    eng = PairEngine(dev, P, 480, 640)
+    eng = PairEngine(dev, P, 480, 640, sp_state_dict=oracle.synthetic_weights("superpoint"), lg_state_dict=oracle.synthetic_weights("lightglue"))
     kp = torch.zeros(2 * P, cap, 2, device=dev); ds = torch.zeros(2 * P, cap, 256, device=dev)
     counts = torch.zeros(2 * P, dtype=torch.int32, device=dev)
     for p, r in enumerate(ref):
@@ -93,10 +95,11 @@ def test_engine_lightglue_on_oracle_features(dev, stream):
 
 def test_engine_device_path_equals_host_path(dev, stream):
     """match_device (HBM-resident inputs: the timed `value`) and match_host (the `e2e` leg) give the same answer."""
+    import oracle
     from imcui_b200.engine import PairEngine
     imgs, _ = stream
     P = 4
-    eng = PairEngine(dev, P, 480, 640)
+    eng = PairEngine(dev, P, 480, 640, sp_state_dict=oracle.synthetic_weights("superpoint"), lg_state_dict=oracle.synthetic_weights("lightglue"))
     eng.h_images.copy_(torch.from_numpy(imgs[: 2 * P]))
     hm, _, hk, hc, hstop = (t.clone() for t in eng.match_host())
     sp, lg = eng.match_device(eng.to_float(eng.h_images.to(dev)))
@@ -109,6 +112,7 @@ def test_pair_stream_from_rgb_frames_equals_the_registry_path(dev, stream):
     """PairStream (double-buffered H2D / compute / D2H over three streams, buffers reused every other batch) on decoded RGB
     frames == the plugin path one pair at a time (extract -> match_images) on the same frames: identical matched keypoints
     in original-frame coordinates; and batch i's record is not disturbed by batches i+1, i+2 in flight."""
+    import oracle
     from imcui_b200.engine import PairEngine, PairStream
     from imcui_b200.hloc import extract_features, match_features
     from imcui_b200.ui import utils as U
@@ -117,13 +121,15 @@ def test_pair_stream_from_rgb_frames_equals_the_registry_path(dev, stream):
     P, NBATCH = 2, 5
     rgb = synth.to_rgb(imgs[: 2 * P * NBATCH])                                     # [20,480,640,3]
     pre = {"grayscale": True, "resize_max": 1600, "dfactor": 8}
-    eng = PairEngine(dev, P, 480, 640, frame_shape=(480, 640, 3), pre_conf=pre)
+    eng = PairEngine(dev, P, 480, 640, sp_state_dict=oracle.synthetic_weights("superpoint"), lg_state_dict=oracle.synthetic_weights("lightglue"), frame_shape=(480, 640, 3), pre_conf=pre)
     batches = [torch.from_numpy(rgb[2 * P * b: 2 * P * (b + 1)]).pin_memory() for b in range(NBATCH)]
     recs = []
     for rec in PairStream(eng).run(iter(batches)):
         recs.append({k: v.clone() for k, v in rec.items()})
     assert len(recs) == NBATCH
     conf = U.get_matcher_zoo({"x": {"matcher": "superpoint-lightglue", "feature": "superpoint_max", "dense": False, "standalone": False}})["x"]
+    conf["feature"] = {**conf["feature"], "model": {**conf["feature"]["model"], "state_dict": oracle.synthetic_weights("superpoint")}}
+    conf["matcher"] = {**conf["matcher"], "model": {**conf["matcher"]["model"], "state_dict": oracle.synthetic_weights("lightglue")}}
     ext, mat = U.get_feature_model(conf["feature"], dev), U.get_model(conf["matcher"], dev)
     ext.conf.update(SP_CONF)
     for b in (0, 3, 4):

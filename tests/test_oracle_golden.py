@@ -1,5 +1,6 @@
 """Pin the CPU oracle (oracle/) against fixtures produced by the unmodified reference modules
-(tools/make_golden.py).  CPU only."""
+(tools/make_golden.py) and, for the networks that run on synthetic parameters (SuperPoint, LightGlue, SuperGlue), against
+the oracle's own outputs on the stored inputs (tools/make_golden_synth.py).  CPU only."""
 import numpy as np
 import pytest
 import torch
@@ -8,7 +9,7 @@ import oracle
 from oracle import lightglue as olg
 from oracle import matchers as om
 from oracle import superpoint as osp
-from conftest import ROOT, lg_pair_from_source, match_f1
+from conftest import ROOT, compressed_descriptors, lg_pair_from_source, match_f1
 
 SP_CONFS = {
     "api": {"nms_radius": 3, "max_keypoints": 1024, "keypoint_threshold": 0.015, "remove_borders": 4},
@@ -20,44 +21,46 @@ SP_CONFS = {
 
 @pytest.mark.parametrize("case,confs", [("sp_real", ["api", "max1024", "nocap"]), ("sp_synth", ["max1024", "max2048"])])
 def test_superpoint_oracle_matches_reference(golden, case, confs):
-    g = golden(case)
-    w = oracle.load_weights("superpoint_v1.pt")
+    g, s = golden(case), golden("sp_sw")
+    w = oracle.synthetic_weights("superpoint")
     images = torch.from_numpy(g["images"])
     for c in confs:
         for b in range(images.shape[0]):
             out = osp.forward(w, images[b:b + 1], SP_CONFS[c])
+            pre = f"{case}/{c}/{b}/"
             # keypoint set + order bit-exact, scores/descriptors to 1e-5 (same machine class: ~0)
-            assert np.array_equal(out["keypoints"][0].numpy().astype(np.int16), g[f"{c}/{b}/keypoints"]), (case, c, b)
-            np.testing.assert_allclose(out["scores"][0].numpy(), g[f"{c}/{b}/scores"], atol=1e-5)
-            np.testing.assert_allclose(out["descriptors"][0].numpy(), g[f"{c}/{b}/descriptors"], atol=1e-4)
+            assert np.array_equal(out["keypoints"][0].numpy().astype(np.int16), s[pre + "keypoints"]), (case, c, b)
+            np.testing.assert_allclose(out["scores"][0].numpy(), s[pre + "scores"], atol=1e-5)
+            np.testing.assert_allclose(out["descriptors"][0].numpy()[:, s[pre + "desc_cols"]], s[pre + "descriptors"], atol=1e-4)
 
 
 def test_superpoint_oracle_fix_sampling(golden):
-    """oracle.sample_descriptors_fix_sampling against the unmodified reference plugin with fix_sampling=True."""
-    g = golden("sp_fix")
-    w = oracle.load_weights("superpoint_v1.pt")
+    """oracle.sample_descriptors_fix_sampling (fix_sampling=True) on the sp_fix images."""
+    g, s = golden("sp_fix"), golden("sp_sw")
+    w = oracle.synthetic_weights("superpoint")
     conf = {"nms_radius": 3, "max_keypoints": 256, "keypoint_threshold": 0.005, "remove_borders": 4, "fix_sampling": True}
     images = torch.from_numpy(g["images"])
     for b in range(images.shape[0]):
         out = osp.forward(w, images[b:b + 1], conf)
-        assert np.array_equal(out["keypoints"][0].numpy().astype(np.int16), g[f"{b}/keypoints"])
-        np.testing.assert_allclose(out["descriptors"][0].numpy(), g[f"{b}/descriptors"], atol=1e-4)
+        cols = s[f"fix/{b}/desc_cols"]
+        assert np.array_equal(out["keypoints"][0].numpy().astype(np.int16), s[f"fix/{b}/keypoints"])
+        np.testing.assert_allclose(out["descriptors"][0].numpy()[:, cols], s[f"fix/{b}/descriptors"], atol=1e-4)
         plain = osp.forward(w, images[b:b + 1], {**conf, "fix_sampling": False})
-        assert np.abs(plain["descriptors"][0].numpy() - g[f"{b}/descriptors"]).max() > 1e-2
+        assert np.abs(plain["descriptors"][0].numpy()[:, cols] - s[f"fix/{b}/descriptors"]).max() > 1e-2
 
 
 def test_superpoint_oracle_dense_maps(golden):
-    g = golden("sp_real")
-    w = oracle.load_weights("superpoint_v1.pt")
+    g, s = golden("sp_real"), golden("sp_sw")
+    w = oracle.synthetic_weights("superpoint")
     out = osp.forward(w, torch.from_numpy(g["images"]), SP_CONFS["api"], return_dense=True)
     for b in range(2):
-        np.testing.assert_allclose(out["dense_scores"][b].numpy(), g[f"dense/{b}/scores"], atol=2e-6)
-        assert np.array_equal(out["nms_scores"][b].numpy() > 0, g[f"dense/{b}/nms3"] > 0)
-        np.testing.assert_allclose(out["dense_descriptors"][b, :, ::4, ::4].numpy(), g[f"dense/{b}/desc_sub"], atol=1e-5)
+        np.testing.assert_allclose(out["dense_scores"][b].numpy().ravel()[s[f"dense/{b}/idx"]], s[f"dense/{b}/scores"], atol=2e-6)
+        assert np.array_equal(np.packbits(out["nms_scores"][b].numpy().ravel() > 0), s[f"dense/{b}/nms3_bits"])
+        np.testing.assert_allclose(out["dense_descriptors"][b, :, ::16, ::16].numpy(), s[f"dense/{b}/desc_sub"], atol=1e-5)
 
 
 def test_superpoint_oracle_rejects_bad_max_keypoints():
-    w = oracle.load_weights("superpoint_v1.pt")
+    w = oracle.synthetic_weights("superpoint")
     with pytest.raises(ValueError):
         osp.forward(w, torch.zeros(1, 1, 16, 16), {"max_keypoints": 0})
 
@@ -73,7 +76,7 @@ MODES = {
 @pytest.mark.parametrize("mode", ["full", "cuda", "cpu"])
 def test_lightglue_oracle_matches_reference(golden, case, mode):
     g = golden(case)
-    w = oracle.load_weights("superpoint_lightglue.pt")
+    w = oracle.synthetic_weights("lightglue")
     for p, src in enumerate(g["sources"]):
         k0, d0, k1, d1 = lg_pair_from_source(golden, src)
         out = olg.forward(w, torch.from_numpy(k0)[None], torch.from_numpy(d0).t().contiguous()[None],
@@ -88,7 +91,7 @@ def test_lightglue_oracle_matches_reference(golden, case, mode):
 
 
 def _lg_proj_weights(g):
-    w = dict(oracle.load_weights("superpoint_lightglue.pt"))
+    w = dict(oracle.synthetic_weights("lightglue"))
     w["input_proj.weight"], w["input_proj.bias"] = torch.from_numpy(g["input_proj_w"]), torch.from_numpy(g["input_proj_b"])
     return w
 
@@ -98,9 +101,9 @@ def test_lightglue_input_proj_oracle_matches_reference(golden):
     g = golden("lg_proj")
     w = _lg_proj_weights(g)
     for p, src in enumerate(g["sources"]):
-        k0, _, k1, _ = lg_pair_from_source(golden, src)
-        out = olg.forward(w, torch.from_numpy(k0)[None], torch.from_numpy(g[f"{p}/descriptors0"])[None],
-                          torch.from_numpy(k1)[None], torch.from_numpy(g[f"{p}/descriptors1"])[None], MODES["cuda"])
+        k0, d0, k1, d1 = lg_pair_from_source(golden, src)
+        c0, c1 = (torch.from_numpy(compressed_descriptors(d, g["input_proj_w"]))[None] for d in (d0, d1))
+        out = olg.forward(w, torch.from_numpy(k0)[None], c0, torch.from_numpy(k1)[None], c1, MODES["cuda"])
         assert out["stop"] == int(g[f"{p}/stop"])
         assert np.array_equal(out["matches0"][0].numpy(), g[f"{p}/matches0"])
         np.testing.assert_allclose(out["matching_scores0"][0].numpy(), g[f"{p}/matching_scores0"], atol=1e-4)
@@ -113,7 +116,7 @@ def test_aliked_lightglue_fitted_input_proj_oracle_matches_reference(golden):
     g = golden("aliked_lg")
     w = _lg_proj_weights(g)
     for p in range(len(g["eval_seeds"])):
-        t = lambda n: torch.from_numpy(g[f"{p}/{n}"])[None]
+        t = lambda n: torch.from_numpy(g[f"{p}/{n}"].astype(np.float32))[None]
         out = olg.forward(w, t("keypoints0"), t("descriptors0"), t("keypoints1"), t("descriptors1"), MODES["cuda"])
         assert out["stop"] == int(g[f"{p}/stop"])
         m = out["matches0"][0].numpy()
@@ -132,10 +135,10 @@ def test_lightglue_scale_ori_oracle_matches_reference(golden):
     w = _lg_proj_weights(g)
     w["posenc.Wr.weight"] = torch.from_numpy(g["posenc_wr"])
     for p, src in enumerate(g["sources"]):
-        k0, _, k1, _ = lg_pair_from_source(golden, src)
+        k0, d0, k1, d1 = lg_pair_from_source(golden, src)
+        c0, c1 = (torch.from_numpy(compressed_descriptors(d, g["input_proj_w"]))[None] for d in (d0, d1))
         so = tuple(torch.from_numpy(g[f"{p}/{n}"])[None] for n in ("scales0", "oris0", "scales1", "oris1"))
-        out = olg.forward(w, torch.from_numpy(k0)[None], torch.from_numpy(g[f"{p}/descriptors0"])[None],
-                          torch.from_numpy(k1)[None], torch.from_numpy(g[f"{p}/descriptors1"])[None], MODES["cuda"], scale_ori=so)
+        out = olg.forward(w, torch.from_numpy(k0)[None], c0, torch.from_numpy(k1)[None], c1, MODES["cuda"], scale_ori=so)
         assert out["stop"] == int(g[f"{p}/stop"])
         assert np.array_equal(out["matches0"][0].numpy(), g[f"{p}/matches0"])
         np.testing.assert_allclose(out["matching_scores0"][0].numpy(), g[f"{p}/matching_scores0"], atol=1e-4)
@@ -155,7 +158,7 @@ def _sg_data(golden, src):
 def test_superglue_oracle_matches_reference(golden, iters):
     from oracle import superglue as osg
     g = golden("sg")
-    w = oracle.load_weights("superglue_outdoor.pt")
+    w = oracle.synthetic_weights("superglue")
     for p, src in enumerate(g["sources"]):
         out = osg.forward(w, _sg_data(golden, src), sinkhorn_iterations=iters, match_threshold=0.2)
         pre = f"it{iters}/{p}/"

@@ -85,6 +85,7 @@ def test_export_features_and_match_from_paths(tmp_path):
     """Files written by the batched exporters == what the reference's per-image / per-pair loops store: keypoints in the original
     frame as fp16, descriptors fp16, matches0 int16 equal to the single-pair plugin result on the stored features."""
     import cv2
+    import oracle
     from imcui_b200.hloc import extractors, matchers, pairs_stream as ps
     from imcui_b200.hloc.configs import confs_dict
     from imcui_b200.hloc.utils import io
@@ -104,7 +105,8 @@ def test_export_features_and_match_from_paths(tmp_path):
     big = cv2.resize(synth.make_pair(7, 480, 640)[0], (1300, 975), interpolation=cv2.INTER_LINEAR)
     cv2.imwrite(str(root / "big.png"), big)                                  # larger than resize_max: area-resized to 1024x768
     names.append("big.png")
-    econf = {"output": "feats-superpoint-n1024-r1024", "model": {**confs_dict["extractors"]["superpoint_aachen"]["model"], "max_keypoints": 1024},
+    econf = {"output": "feats-superpoint-n1024-r1024", "model": {**confs_dict["extractors"]["superpoint_aachen"]["model"], "max_keypoints": 1024,
+                                                                  "state_dict": oracle.synthetic_weights("superpoint")},
              "preprocessing": {"grayscale": True, "resize_max": 1024}}
     fpath = ps.export_features(econf, root, feature_path=tmp_path / "feats.imw", batch=4)
     assert sorted(io.list_h5_names(fpath)) == sorted(names)
@@ -129,6 +131,8 @@ def test_export_features_and_match_from_paths(tmp_path):
     (tmp_path / "pairs.txt").write_text("".join(f"db/{s}a.png db/{s}b.png\n" for s in range(3)) + "db/0b.png db/0a.png\ndb/0a.png big.png\n")
     for mname, plugin in (("NN-mutual", "nearest_neighbor"), ("superpoint-lightglue", "lightglue")):
         mconf = confs_dict["matchers"][mname]
+        if plugin == "lightglue":
+            mconf = {**mconf, "model": {**mconf["model"], "state_dict": oracle.synthetic_weights("lightglue")}}
         mpath = ps.match_from_paths(mconf, tmp_path / "pairs.txt", tmp_path / f"m_{plugin}.imw", fpath, fpath, batch=3)
         model = dynamic_load(matchers, plugin)(mconf["model"]).eval().to(dev)
         with open_store(mpath, "r") as ms, open_store(fpath, "r") as fs:

@@ -50,7 +50,7 @@ def sp_features(dev, P, cap=1024):
 def row_superglue(dev, iters):
     P = 16
     sp = sp_features(dev, P)
-    sd = torch.load(str(ROOT / "weights/superglue_outdoor.pt"), map_location="cpu")
+    sd = synth_weights.superglue_random_weights(0)
     w = {k: v.to(dev) for k, v in ops.sg_pack_weights(sd).items()}
     wh = torch.tensor([[640, 480]] * (2 * P), dtype=torch.int32, device=dev)
     counts = sp["counts"][0].contiguous()
@@ -139,7 +139,7 @@ def row_config4(dev, iters):
     P, cap = 32, 1024
     aw = {k: v.to(dev) for k, v in ops.aliked_pack_weights(synth_weights.aliked_random_weights(0)).items()}
     g = np.load(ROOT / "tests/golden/lg_proj.npz")
-    sd = dict(torch.load(str(ROOT / "weights/superpoint_lightglue.pt"), map_location="cpu"))
+    sd = synth_weights.lightglue_random_weights(0)
     sd["input_proj.weight"], sd["input_proj.bias"] = torch.from_numpy(g["input_proj_w"]), torch.from_numpy(g["input_proj_b"])
     lw = {k: v.to(dev) for k, v in ops.lg_pack_weights(sd, 9).items()}
     a, b = synth.make_pair_batch(list(range(P)))

@@ -12,7 +12,7 @@ import oracle
 from oracle import superpoint as osp
 from imcui_b200.utils import synth
 torch.set_num_threads(8)
-ws = oracle.load_weights("superpoint_v1.pt")
+ws = oracle.synthetic_weights("superpoint")
 CONF = {"nms_radius": 3, "keypoint_threshold": 0.005, "max_keypoints": -1, "remove_borders": 4}
 
 def split_f16(x):
