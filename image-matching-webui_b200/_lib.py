@@ -67,6 +67,14 @@ class AlikedConf(C.Structure):
     _fields_ = [("detection_threshold", C.c_float), ("max_num_keypoints", C.c_int), ("nms_radius", C.c_int)]
 
 
+IMW_SIFT_MAX_TAPS = 64
+
+
+class SiftConf(C.Structure):
+    _fields_ = [("n_octave_layers", C.c_int), ("contrast_threshold", C.c_float), ("edge_threshold", C.c_float), ("sigma", C.c_double),
+                ("max_keypoints", C.c_int), ("nms_radius", C.c_int), ("rootsift", C.c_int)]
+
+
 class LoftrConv(C.Structure):
     _fields_ = [("w", C.c_void_p), ("b", C.c_void_p), ("cin", C.c_int), ("cout", C.c_int), ("ksize", C.c_int), ("stride", C.c_int)]
 
@@ -128,6 +136,13 @@ def lib():
         L.imw_aliked_forward.argtypes = [C.POINTER(AlikedWeights), C.POINTER(AlikedConf), C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                          C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_size_t, C.c_void_p]
+        L.imw_sift_plan.restype = C.c_int
+        L.imw_sift_plan.argtypes = [C.POINTER(SiftConf), C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.imw_sift_workspace_bytes.restype = C.c_size_t
+        L.imw_sift_workspace_bytes.argtypes = [C.POINTER(SiftConf), C.c_int, C.c_int, C.c_int]
+        L.imw_sift_forward.restype = C.c_int
+        L.imw_sift_forward.argtypes = [C.POINTER(SiftConf), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 8 + \
+                                      [C.c_size_t, C.c_void_p]
         L.imw_loftr_workspace_bytes.restype = C.c_size_t
         L.imw_loftr_workspace_bytes.argtypes = [C.c_int] * 4
         L.imw_loftr_workspace_bytes_hw.restype = C.c_size_t

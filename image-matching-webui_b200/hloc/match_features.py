@@ -30,7 +30,8 @@ def pair_inputs(feat0, feat1):
         data["descriptors" + side] = desc.unsqueeze(0) if desc.dim() == 2 else desc
         for extra in ("scales", "oris"):
             if extra in f:
-                data[extra + side] = f[extra]
+                x = f[extra]
+                data[extra + side] = _first(x)[None] if isinstance(x, (list, tuple)) else x
     return data
 
 

@@ -478,6 +478,71 @@ def aliked_forward(bufs, image, conf, cap, debug=False):
 
 
 # ---------------------------------------------------------------------------------------------------
+# SIFT
+# ---------------------------------------------------------------------------------------------------
+def sift_conf_struct(conf):
+    """conf keys: n_octave_layers, contrast_threshold, edge_threshold, sigma, max_keypoints (<= 0: all),
+    nms_radius (None or 0), rootsift"""
+    nms = conf.get("nms_radius")
+    return L.SiftConf(int(conf["n_octave_layers"]), float(conf["contrast_threshold"]), float(conf["edge_threshold"]),
+                      float(conf.get("sigma", 1.6)), int(conf["max_keypoints"] or 0), -1 if nms is None else int(nms),
+                      int(bool(conf["rootsift"])))
+
+
+def sift_plan(conf, height, width):
+    """Host-only: (octave count, [(ksize, taps as float32 numpy)] per pyramid layer; entry 0 blurs the doubled base)."""
+    import numpy as np
+    c = sift_conf_struct(conf)
+    n_layers = c.n_octave_layers + 3
+    n_oct = C.c_int()
+    ks = (C.c_int * n_layers)()
+    taps = np.zeros((n_layers, L.IMW_SIFT_MAX_TAPS), np.float32)
+    L.check(L.lib().imw_sift_plan(C.byref(c), height, width, C.addressof(n_oct), C.addressof(ks), taps.ctypes.data))
+    return n_oct.value, [(ks[i], taps[i, :ks[i]].copy()) for i in range(n_layers)]
+
+
+def sift_pyramid_shapes(conf, height, width):
+    """[(octave, layers, h, w)] of the Gaussian pyramid (octave -1 is the doubled image)."""
+    n_oct, _ = sift_plan(conf, height, width)
+    lay = int(conf["n_octave_layers"]) + 3
+    return [(o - 1, lay, (2 * height) >> o, (2 * width) >> o) for o in range(n_oct)]
+
+
+def sift_forward(image, conf, cap, debug=False):
+    """image [B,1,H,W] fp32 CUDA in [0,1].  Returns batch buffers in descending response order: keypoints [B,cap,2],
+    scores / scales / oris [B,cap], descriptors [B,cap,128], counts [2,B] int32 (written, total; total -1 = internal
+    capacity exceeded) (+ pyramid: a list of [B, L+3, h, w] per octave with debug)."""
+    L.require_cuda(image, "sift_forward(image)")
+    assert image.dim() == 4 and image.shape[1] == 1 and image.dtype == torch.float32
+    image = image.contiguous()
+    B, _, H, W = image.shape
+    dev = image.device
+    c = sift_conf_struct(conf)
+    out = {"keypoints": torch.empty(B, cap, 2, device=dev), "scores": torch.empty(B, cap, device=dev),
+           "scales": torch.empty(B, cap, device=dev), "oris": torch.empty(B, cap, device=dev),
+           "descriptors": torch.empty(B, cap, 128, device=dev), "counts": torch.empty(2, B, dtype=torch.int32, device=dev)}
+    shapes = sift_pyramid_shapes(conf, H, W) if debug else []
+    pyr = torch.empty(B, sum(l * h * w for _, l, h, w in shapes), device=dev) if debug else None
+    lib = L.lib()
+    nbytes = lib.imw_sift_workspace_bytes(C.byref(c), B, H, W)
+    if nbytes == 0:
+        L.check(lib.imw_sift_plan(C.byref(c), H, W, None, None, None))
+    ws = L.workspaces.get(dev, nbytes, "sift")
+    with torch.cuda.device(dev):
+        rc = lib.imw_sift_forward(C.byref(c), B, H, W, L.ptr(image), cap, L.ptr(out["keypoints"]), L.ptr(out["scores"]),
+                                  L.ptr(out["scales"]), L.ptr(out["oris"]), L.ptr(out["descriptors"]), L.ptr(out["counts"]),
+                                  L.ptr(pyr), L.ptr(ws), ws.numel(), L.stream_ptr(dev))
+    L.check(rc)
+    if debug:
+        levels, off = [], 0
+        for _, l, h, w in shapes:
+            levels.append(pyr[:, off:off + l * h * w].view(B, l, h, w))
+            off += l * h * w
+        out["pyramid"] = levels
+    return out
+
+
+# ---------------------------------------------------------------------------------------------------
 # LoFTR
 # ---------------------------------------------------------------------------------------------------
 def _pad_to(n, m=64):

@@ -292,6 +292,37 @@ int imw_aliked_forward(const imw_aliked_weights* weights, const imw_aliked_conf*
                        float* dbg_score_map, float* dbg_feature_map, void* workspace, size_t workspace_bytes, imw_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * SIFT extractor.
+ * Replaces: hloc/extractors/sift.py (opencv backend) -> cv2.SIFT_create(...).detectAndCompute on uint8(trunc(x * 255))
+ * with firstOctave -1, then the LightGlue wrapper glue (lightglue/sift.py): filter_dog_point (nms_radius 0), top-k on the
+ * response, RootSIFT.  No weights.
+ * ---------------------------------------------------------------------------------------------- */
+#define IMW_SIFT_MAX_TAPS 64
+
+typedef struct {
+  int n_octave_layers;      /* cv2 nOctaveLayers (the wrapper passes its num_octaves = 4 here) */
+  float contrast_threshold; /* cv2 contrastThreshold (wrapper: detection_threshold) */
+  float edge_threshold;     /* cv2 edgeThreshold */
+  double sigma;             /* 1.6 (a double, as cv::SIFT keeps it: the pyramid sigmas are computed from it in double) */
+  int max_keypoints;        /* cv2 nfeatures and the wrapper's top-k; <= 0: all */
+  int nms_radius;           /* -1: no pixel filter (None), 0: filter_dog_point's one-keypoint-per-pixel rule */
+  int rootsift;             /* 1: RootSIFT descriptors (unit L2 norm), 0: cv2's integer-valued descriptors */
+} imw_sift_conf;
+
+/* host-only: octave count of a height x width input and the Gaussian kernels of the pyramid (ksizes [L+3], taps
+ * [L+3][IMW_SIFT_MAX_TAPS]; index 0 is the blur of the doubled base image).  Any output may be NULL. */
+int imw_sift_plan(const imw_sift_conf* conf, int height, int width, int* n_octaves, int* ksizes, float* taps);
+size_t imw_sift_workspace_bytes(const imw_sift_conf* conf, int batch, int height, int width);
+/* images [B][H][W] fp32 gray in [0,1] (H, W <= 4096).  Outputs in descending response order: keypoints [B][cap][2] (x, y),
+ * scores [B][cap] (response), scales [B][cap] (size), oris [B][cap] (radians), descriptors [B][cap][128];
+ * counts [2B]: [0,B) written, [B,2B) keypoints the reference returns (> cap: call again with a larger cap; -1: more
+ * extrema than the internal per-image capacity).  dbg_pyramid (nullable): the Gaussian layers, per image octave after octave,
+ * (L+3) layers of (2H >> o) x (2W >> o) each. */
+int imw_sift_forward(const imw_sift_conf* conf, int batch, int height, int width, const float* images, int cap, float* keypoints,
+                     float* scores, float* scales, float* oris, float* descriptors, int* counts, float* dbg_pyramid,
+                     void* workspace, size_t workspace_bytes, imw_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * LoFTR dense matcher.
  * Replaces: hloc/matchers/loftr.py:41-71 -> kornia.feature.LoFTR == third_party/SE2LoFTR/src/loftr/loftr.py:29-75
  * (ResNet-FPN backbone, coarse linear-attention transformer, dual-softmax coarse matching, fine refinement).
